@@ -5,11 +5,15 @@ Headline (BASELINE.json `metric`, configs[1]; configs[3] for N > 1): Spex+, 32 m
 Second block `pbsrnn` (the other model the metric's target names; configs[2]): pBSRNN, bsrnn.yaml network, 16 rows per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows 32] [--bsrnn-rows 16]
+                  [--dump-outputs DIR]
 
 A "step" = forward + loss (Spex+: 0.8/0.1/0.1 SI-SDR + 0.5 CE; pBSRNN: SI-SDR) + backward + gradient all-reduce (N > 1) +
 per-tensor clip + Adam, the loop body of the reference Executor.train (wesep/utils/executor.py:70-134).
 Prints ONE JSON line on rank 0.  `value`: inputs already resident in HBM; `e2e`: same step through
 the public API from pinned host buffers (H2D every step, D2H of the loss every step).
+--dump-outputs DIR: after the JSON line, rank 0 writes what the last timed (resident) step of each model block left to its
+caller as DIR/<block>_{loss,grads}.npy (see `step_outputs`).  That step starts from the seeded initial state (`time_steps`),
+so its inputs depend on the arguments only and two builds run with the same arguments can be compared array for array.
 `roofline` describes the kernel with the LARGEST share of the timed step (shares from one CUPTI pass of a step inside this
 run), `roofline.step` the whole step against the HBM roofline SURVEY.md 8d says binds it.
 """
@@ -49,6 +53,7 @@ BSRNN_FBANK_FRAMES = 398        # 1 + (64000 - 400) // 160 frames of 25 ms / 10 
 SPEX_BYTES_PER_ROW = 6.4e9      # algorithmic HBM bytes per row per train step (SURVEY.md 8d: 32 x 190 MB + 0.35 GB)
 SPEX_FLOPS_PER_ROW = 396e9      # algorithmic flops per row per train step (132 GFLOP forward x 3)
 BSRNN_FLOPS_PER_ROW = 1.02e12   # (340 GFLOP forward x 3)
+DUMP_SAMPLE = 1 << 20           # --dump-outputs: at most this many elements per array (4 MiB fp32; 4 blocks = 16 MiB)
 
 
 def peaks():
@@ -155,7 +160,7 @@ def run_reference(args, rank):
         return
     threads = cpu_threads()
     rows = max(2, args.ref_rows)                    # >= 2 rows so the BatchNorm of the speaker encoder sees a batch
-    steps, warm = max(1, min(args.steps, 3)), max(0, min(args.warmup, 1))
+    steps, warm = args.steps, max(0, min(args.warmup, 1))
     val, med, loss = cpu_train_rows_per_s(rows, steps, warm, threads)
     sample = (f"{rows} rows x {T_SAMPLES} samples per step; ran {warm} warm-up + {steps} timed steps (median {med:.2f} s); "
               f"oracle port (plain torch fp32) on {threads} threads of {os.cpu_count()} host cores ({cpu_model_name()})")
@@ -286,21 +291,30 @@ def gpu_eager_baseline(n, dev):
     return out
 
 
-def time_steps(one, warmup, steps, barrier, world, dev):
+def time_steps(one, warmup, steps, barrier, world, dev, restore=None):
+    """`warmup` untimed steps, then `steps` timed ones.  `restore()` runs between the two timed windows, right before the last
+    step: it puts the model back into the seeded state it started from, so what that step computes depends on the arguments
+    only.  (The kernels accumulate in fp32 with atomics, so every step is reproducible to rounding; Adam's first updates move
+    each element by about +-lr according to its gradient's sign, which would turn that rounding into differences of order lr
+    after a few steps.)"""
     from wesep_b200 import _lib
     import torch.distributed as dist
     for _ in range(warmup):
         one()
     barrier()
     l0 = _lib.launch_count()
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record()
-    last = None
-    for _ in range(steps):
-        last = one()
-    e.record()
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+    ev[0].record()
+    for _ in range(steps - 1):
+        one()
+    ev[1].record()
+    if restore is not None:
+        restore()
+    ev[2].record()
+    last = one()
+    ev[3].record()
     barrier()
-    ms = s.elapsed_time(e)
+    ms = ev[0].elapsed_time(ev[1]) + ev[2].elapsed_time(ev[3])
     launches = _lib.launch_count() - l0
     if world > 1:
         tt = torch.tensor([ms], device=dev)
@@ -309,12 +323,43 @@ def time_steps(one, warmup, steps, barrier, world, dev):
     return ms, launches, float(last)
 
 
-def run_pbsrnn(args, rank, world, dev, pk, barrier):
+def _dump_sample(x):
+    """x (flat, on the device) as an fp32 host array; beyond DUMP_SAMPLE elements, the same seeded sample of indices for a
+    given length."""
+    if x.numel() > DUMP_SAMPLE:
+        import numpy as np
+        idx = np.sort(np.random.default_rng(0).choice(x.numel(), DUMP_SAMPLE, replace=False))
+        x = x[torch.from_numpy(idx).to(x.device)]
+    return x.float().cpu().numpy()
+
+
+def step_outputs(opt, loss):
+    """What a train step computes for its caller: the loss and the gradients the optimizer applied (in parameter order).  The
+    updated parameters are left out: Adam's step from the seeded state moves every element by about +-lr by the sign of its
+    gradient, and for elements whose gradient is at rounding level (e.g. the exactly-zero decoder-bias gradients of the
+    shift-invariant SI-SDR) that sign is itself rounding."""
+    import numpy as np
+    with torch.no_grad():
+        grads = torch.cat([p.grad.reshape(-1) for p in opt.arena.params])
+    return dict(loss=np.array([loss], np.float64), grads=_dump_sample(grads))
+
+
+def write_outputs(out_dir, blocks):
+    """blocks: {block name: step_outputs(...)} -> out_dir/<block>_<array>.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for block, arrays in blocks.items():
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, f"{block}_{name}.npy"), a)
+
+
+def run_pbsrnn(args, rank, world, dev, pk, barrier, dumps):
     """BASELINE config 3: pBSRNN train step, 4 s @ 16 kHz, 16 rows per GPU, bsrnn.yaml network (speaker embeddings as input)."""
     import numpy as np
     from wesep_b200 import _lib, ops, synth
     from wesep_b200.distributed import GradAllReducer, broadcast_params
     from wesep_b200.models import get_model
+    from wesep_b200.utils.executor import restore_train_state, snapshot_train_state
     from wesep_b200.utils.optim import FusedClipAdam
     n = args.bsrnn_rows
     torch.manual_seed(42 + rank)
@@ -359,10 +404,16 @@ def run_pbsrnn(args, rank, world, dev, pk, barrier):
             loss = graphed(batch)                                   # copies the batch (pinned host or device) into the static inputs
             return loss.item() if read_loss else loss
 
-    ms_res, launches, loss_res = time_steps(lambda: step(resident, False), args.warmup, args.steps, barrier, world, dev)
+    seed = snapshot_train_state(model, opt)
+
+    def restore():
+        restore_train_state(model, opt, seed)
+    ms_res, launches, loss_res = time_steps(lambda: step(resident, False), args.warmup, args.steps, barrier, world, dev, restore)
+    if args.dump_outputs and rank == 0:
+        dumps["pbsrnn"] = step_outputs(opt, loss_res)
     if graphed is not None:
         launches = graphed.launches_per_step * args.steps
-    ms_e2e, _, loss_e2e = time_steps(lambda: step(host, True), 1, args.steps, barrier, world, dev)
+    ms_e2e, _, loss_e2e = time_steps(lambda: step(host, True), 1, args.steps, barrier, world, dev, restore)
     if rank != 0:
         step(resident, False)          # the CUPTI pass below is one more COLLECTIVE step: every rank takes part
         barrier()
@@ -406,12 +457,13 @@ def run_pbsrnn(args, rank, world, dev, pk, barrier):
                 top_kernels=[dict(kernel=k[:70], share=v[1] / tot, count=v[0]) for k, v in top])
 
 
-def run_extra(args, dev, which):
+def run_extra(args, dev, which, dumps):
     """Further blocks (single GPU only): pDPCCN (SURVEY.md 8 row a23) and TF-GridNet (row a24, BASELINE config 5) train steps on
     the recipe networks verbatim (jointly trained ResNet34 on fbank features), 4 s @ 16 kHz, eager launches."""
     import numpy as np
     from wesep_b200 import _lib, ops, synth
     from wesep_b200.models import get_model
+    from wesep_b200.utils.executor import restore_train_state, snapshot_train_state
     from wesep_b200.utils.optim import FusedClipAdam
     n = args.dpccn_rows if which == "DPCCN" else args.tfgridnet_rows
     torch.manual_seed(42)
@@ -433,7 +485,7 @@ def run_extra(args, dev, which):
         opt.step()
         return losses[0].item() if read_loss else losses[0]
 
-    K = max(1, min(args.steps, 5))
+    K = args.steps
 
     def sync():
         torch.cuda.synchronize(dev)
@@ -457,8 +509,14 @@ def run_extra(args, dev, which):
         except Exception as ex:                                    # capture is an optimisation: fall back to eager launches
             graphed, graph_error = None, repr(ex)[:200]
             torch.cuda.synchronize(dev)
-    ms_res, launches, loss_res = time_steps(lambda: step(resident, False), 3, K, sync, 1, dev)
-    ms_e2e, _, loss_e2e = time_steps(lambda: step(host, True), 1, K, sync, 1, dev)
+    seed = snapshot_train_state(model, opt)
+
+    def restore():
+        restore_train_state(model, opt, seed)
+    ms_res, launches, loss_res = time_steps(lambda: step(resident, False), 3, K, sync, 1, dev, restore)
+    if args.dump_outputs:
+        dumps[which.lower()] = step_outputs(opt, loss_res)
+    ms_e2e, _, loss_e2e = time_steps(lambda: step(host, True), 1, K, sync, 1, dev, restore)
     if graphed is not None:
         launches = graphed.launches_per_step * K
     agg, tot = kernel_shares(lambda: step(resident, False))
@@ -485,7 +543,7 @@ def run_extra(args, dev, which):
                         ms_per_step=ms_e2e / K),
                gpu_launches=launches, loss=loss_res, loss_e2e=loss_e2e, peak_mem_gb=torch.cuda.max_memory_allocated(dev) / 2 ** 30,
                top_kernels=[dict(kernel=k[:70], share=v[1] / tot, count=v[0]) for k, v in top])
-    del model, opt, resident
+    del model, opt, resident, seed
     torch.cuda.empty_cache()
     return out
 
@@ -494,7 +552,7 @@ def run_ours(args, rank, world, local):
     from wesep_b200 import _lib, synth
     from wesep_b200.distributed import GradAllReducer, broadcast_params
     from wesep_b200.models import get_model
-    from wesep_b200.utils.executor import train_step
+    from wesep_b200.utils.executor import restore_train_state, snapshot_train_state, train_step
     from wesep_b200.utils.lr import exponential_decrease_lr, set_lr
     from wesep_b200.utils.optim import FusedClipAdam
     import torch.distributed as dist
@@ -536,10 +594,17 @@ def run_ours(args, rank, world, local):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_res, launches, loss_res = time_steps(lambda: one(resident, False), args.warmup, args.steps, barrier, world, dev)
+    seed = snapshot_train_state(model, opt)
+
+    def restore():
+        restore_train_state(model, opt, seed)
+    ms_res, launches, loss_res = time_steps(lambda: one(resident, False), args.warmup, args.steps, barrier, world, dev, restore)
+    dumps = {}
+    if args.dump_outputs and rank == 0:
+        dumps["spex"] = step_outputs(opt, loss_res)
     if graphed is not None:                                     # replays do not pass through the host-side counter
         launches = graphed.launches_per_step * args.steps
-    ms_e2e, _, loss_e2e = time_steps(lambda: one(host, True), args.warmup, args.steps, barrier, world, dev)
+    ms_e2e, _, loss_e2e = time_steps(lambda: one(host, True), args.warmup, args.steps, barrier, world, dev, restore)
     clocks_spex = sampler.summary() if sampler else None
     value = n * world * args.steps / (ms_res * 1e-3)
     e2e = n * world * args.steps / (ms_e2e * 1e-3)
@@ -564,23 +629,23 @@ def run_ours(args, rank, world, local):
                                    for k, v in sorted(agg.items(), key=lambda kv: -kv[1][1])[:6]]
     barrier()
     # free the Spex+ state before the second model
-    del model, opt, reducer, resident, graphed
+    del model, opt, reducer, resident, graphed, seed
     torch.cuda.empty_cache()
     pb = None
     if not args.no_pbsrnn:
-        pb = run_pbsrnn(args, rank, world, dev, pk, barrier)
+        pb = run_pbsrnn(args, rank, world, dev, pk, barrier, dumps)
     if rank != 0:
         return
     dp = None
     if world == 1 and not args.no_dpccn:
         try:
-            dp = run_extra(args, dev, "DPCCN")
+            dp = run_extra(args, dev, "DPCCN", dumps)
         except Exception as ex:                                 # extra block: never lose the bench line over it
             dp = dict(error=repr(ex)[:300])
     tg = None
     if world == 1 and not args.no_tfgridnet:
         try:
-            tg = run_extra(args, dev, "TFGridNet")
+            tg = run_extra(args, dev, "TFGridNet", dumps)
         except Exception as ex:
             tg = dict(error=repr(ex)[:300])
     cpu = eager = None
@@ -612,12 +677,14 @@ def run_ours(args, rank, world, local):
         gpu_launches=launches, clocks=clocks_spex, loss=loss_res, loss_e2e=loss_e2e,
         roofline=roof, pbsrnn=pb, dpccn=dp, tfgridnet=tg, cpu_baseline=cpu, gpu_eager_baseline=eager)
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, dumps)
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every model block (and of the --impl reference arm)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=32, help="Spex+ model rows (utterances) per GPU per step")
@@ -632,7 +699,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="pBSRNN block: eager launches instead of a CUDA-graph replay per step")
     ap.add_argument("--cuda-graph", action="store_true",
                     help="capture the whole Spex+ train step in a CUDA graph and time replays (single GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of each block's last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

@@ -1,8 +1,8 @@
 """ORACLE (test infrastructure) — import the REAL reference package from /root/reference.
 
-Only usable in the build container (the GPU box has no /root/reference).  Used by
-tests/golden/make_golden.py and tests/test_oracle_vs_reference.py to pin the restatement
-in oracle/*.py against the reference's own modules.  Nothing is copied: the reference is
+Only usable where the reference tree exists; no test needs it.  Used by the fixture generators
+tests/golden/make_golden*.py to pin the restatement in oracle/*.py against the reference's
+own modules.  Nothing is copied: the reference is
 imported in place through three stub packages (oracle/stubs) for its missing deps.
 """
 import os

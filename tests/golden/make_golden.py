@@ -6,7 +6,7 @@ place through oracle/stubs) on seeded inputs.  Run in the build container only:
 Weights and inputs are NOT stored: both sides regenerate them with
 ``wesep_b200.synth.fill_state_dict_(sd, seed)`` / ``make_batch(seed=...)`` (numpy PCG64,
 machine independent).  Stored: reference outputs, loss parts, per-parameter gradient
-norms / sums (+ full gradients of small tensors).  The reference ships no golden vectors
+norms (+ full gradients of small tensors); every fixture stays under 1 MB.  The reference ships no golden vectors
 of its own (SURVEY.md §4), so these are the pin for oracle/*.py and, through it, for
 the CUDA path.
 """
@@ -34,7 +34,6 @@ def grads_summary(model):
             continue
         g64 = g.double()
         out["gnorm/" + k] = np.float64(g64.norm().item())
-        out["gsum/" + k] = np.float64(g64.sum().item())
         if g.numel() <= 4096:
             out["g/" + k] = g.detach().numpy().copy()
     return out

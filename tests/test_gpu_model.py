@@ -7,15 +7,11 @@ import torch
 from oracle import losses as olosses
 from oracle import optim as ooptim
 from oracle import spexplus as ospex
-from tests.util import cfg_from_args, fixture_inputs, load_fixture, rel_l2
+from tests.util import ZERO_GRAD, cfg_from_args, fixture_inputs, load_fixture, rel_l2
 from wesep_b200 import synth
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-# SI-SDR is invariant to a DC shift of the estimate, so d(loss)/d(decoder bias) is exactly 0 in exact arithmetic:
-# both sides only hold fp32 round-off there (|g| ~ 1e-5..1e-4) and a relative comparison is meaningless.
-import re  # noqa: E402
-ZERO_GRAD = re.compile(r"decoder\.decoder_1d_\d\.bias$")
 
 
 def build_model(args, wseed):

@@ -9,7 +9,7 @@ import torch
 
 from oracle import bsrnn as ob
 from oracle import losses as olosses
-from oracle import ref_loader
+from tests.util import load_layouts
 from wesep_b200 import synth
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -84,19 +84,16 @@ def _load(name):
 
 
 def test_state_dict_layout_matches_reference_order():
-    """The key list (and order: optimizer state and checkpoints depend on it) equals the reference's, when it can be
-    imported (build container); on the GPU box this part is skipped."""
-    if not ref_loader.available():
-        pytest.skip("reference tree not present")
-    ref_loader.import_reference()
-    from wesep.models.bsrnn import BSRNN
+    """The key list (and order: optimizer state and checkpoints depend on it) equals the reference's, as stored from the
+    reference BSRNN in tests/golden/state_dict_layouts.npz (tests/golden/make_golden_layouts.py)."""
+    layouts = load_layouts()
     for fuse, mf in (("multiply", False), ("concat", True)):
         args = dict(spk_emb_dim=256, sr=16000, win=512, stride=128, feature_dim=16, num_repeat=2, use_spk_transform=False,
                     spk_fuse_type=fuse, multi_fuse=mf, joint_training=False)
-        ref = BSRNN(**args).state_dict()
+        ref = [(k, tuple(s)) for k, s in layouts[f"bsrnn/{fuse}/multi_fuse={mf}"]]
         mine = _state_dict_like(args)
-        assert list(ref.keys()) == list(mine.keys())
-        assert all(tuple(ref[k].shape) == tuple(mine[k].shape) for k in ref)
+        assert [k for k, _ in ref] == list(mine.keys())
+        assert all(s == tuple(mine[k].shape) for k, s in ref)
 
 
 @pytest.mark.parametrize("L", [4000, 1023, 512])

@@ -1,6 +1,7 @@
 """Shared helpers for the parity tests (tests may import oracle/)."""
 import json
 import os
+import re
 
 import numpy as np
 import torch
@@ -9,12 +10,22 @@ from oracle import spexplus as ospex
 from wesep_b200 import synth
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# SI-SDR is invariant to a DC shift of the estimate, so d(loss)/d(decoder bias) is exactly 0 in exact arithmetic:
+# both sides only hold fp32 round-off there (|g| ~ 1e-5..1e-4, different with every reduction order, i.e. with the
+# CPU's thread count and vector width) and a relative comparison is meaningless.
+ZERO_GRAD = re.compile(r"decoder\.decoder_1d_\d\.bias$")
 
 
 def load_fixture(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
     meta = json.loads(str(z["meta"]))
     return z, meta
+
+
+def load_layouts():
+    """{"spex/<fuse type>" | "bsrnn/<fuse type>/multi_fuse=<bool>": [[key, shape], ...]}: the reference state_dict layouts
+    (tests/golden/make_golden_layouts.py)."""
+    return json.loads(str(np.load(os.path.join(GOLDEN, "state_dict_layouts.npz"))["layouts"]))
 
 
 def cfg_from_args(args):

@@ -52,6 +52,23 @@ def train_step(model, batch, optimizer, reducer=None, loss_posi=((0, 1, 2), (3,)
     return loss
 
 
+def snapshot_train_state(model, optimizer):
+    """Copies of everything a train step updates: parameters, Adam moments and step counter, module buffers."""
+    return dict(p=optimizer.arena.flat_p.clone(), m=optimizer.exp_avg.clone(), v=optimizer.exp_avg_sq.clone(),
+                step=optimizer.step_count, bufs={k: b.clone() for k, b in model.named_buffers()})
+
+
+def restore_train_state(model, optimizer, snap):
+    """Puts a snapshot_train_state() back in place (same storage, so CUDA graphs keep seeing it)."""
+    with torch.no_grad():
+        optimizer.arena.flat_p.copy_(snap["p"])
+        optimizer.exp_avg.copy_(snap["m"])
+        optimizer.exp_avg_sq.copy_(snap["v"])
+        optimizer.step_count = snap["step"]
+        for k, b in model.named_buffers():
+            b.copy_(snap["bufs"][k])
+
+
 class GraphedStep:
     """A whole train step (zero_grad, forward, loss, backward, clip + Adam) captured ONCE in a CUDA graph and replayed:
     the ~10^3 kernel launches of a step become one graph launch, removing the inter-kernel gaps and all per-step Python /
@@ -71,8 +88,7 @@ class GraphedStep:
         dev = next(model.parameters()).device
         self.static = {k: v.to(dev).clone() for k, v in example_batch.items()}
         optimizer.enable_device_scalars()
-        snap = dict(p=optimizer.arena.flat_p.clone(), m=optimizer.exp_avg.clone(), v=optimizer.exp_avg_sq.clone(),
-                    step=optimizer.step_count, bufs={k: b.clone() for k, b in model.named_buffers()})
+        snap = snapshot_train_state(model, optimizer)
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):                      # warm-up off the default stream, as graph capture requires
@@ -81,22 +97,13 @@ class GraphedStep:
                 self._body()
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
-        self._restore(snap)
+        restore_train_state(model, optimizer, snap)
         self.graph = torch.cuda.CUDAGraph()
         l0 = ops._lib.launch_count()
         with torch.cuda.graph(self.graph):
             self.loss = self._body()
         self.launches_per_step = ops._lib.launch_count() - l0   # kernels of this library inside one replay
-        self._restore(snap)                                # (capture does not execute, but keep the invariant explicit)
-
-    def _restore(self, snap):
-        with torch.no_grad():
-            self.opt.arena.flat_p.copy_(snap["p"])
-            self.opt.exp_avg.copy_(snap["m"])
-            self.opt.exp_avg_sq.copy_(snap["v"])
-            self.opt.step_count = snap["step"]
-            for k, b in self.model.named_buffers():
-                b.copy_(snap["bufs"][k])
+        restore_train_state(model, optimizer, snap)        # (capture does not execute, but keep the invariant explicit)
 
     def _body(self):
         self.opt.zero_grad()
